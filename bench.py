@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's B200 path
   python bench.py --impl reference --gpus N --steps K ...   # the reference's algorithm on host cores
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's results as DIR/*.npy
 
 A step = one pre-training iteration through the public model API: forward (TimeSformer ->
 abstractor -> frozen GPT-3 1.3B -> masked CE), backward (dgrad everywhere, wgrad for the 130 M
@@ -131,10 +132,12 @@ def make_text(G, B, L, vocab, seed, bos=1, pad=0):
     return ids, att
 
 
-def cpu_baseline(port, torch, T, L, Q, iters=1, warmup=1):
+def cpu_baseline(port, torch, T, L, Q, iters=1, warmup=1, cold_cutoff_s=None):
     """The oracle port (fp32, host threads) on a bounded sample: fwd+bwd of ONE sample of the same
     workload, `warmup` untimed + `iters` timed iterations (the first call pays page faults for ~10 GB of
-    weights / saved activations).  Returns (samples/s, threads, description)."""
+    weights / saved activations).  With cold_cutoff_s, a last warm-up iteration slower than that is taken as the
+    only timed one, which keeps an informational baseline within minutes on slow hosts.
+    Returns (samples/s, threads, description)."""
     vcfg = dict(port.VCFG_CLIP_B16, num_frames=T)
     threads = min(os.cpu_count() or 1, 32)   # beyond ~32 threads the small-GEMM torch CPU path slows down
     torch.set_num_threads(threads)
@@ -157,7 +160,7 @@ def cpu_baseline(port, torch, T, L, Q, iters=1, warmup=1):
 
     cold = [one() for _ in range(warmup)]
     note = ""
-    if cold and cold[-1] > 90.0:      # keep the whole run within a few minutes on slow hosts
+    if cold_cutoff_s is not None and cold and cold[-1] > cold_cutoff_s:
         times, note = cold[-1:], " (cold first iteration: the host was too slow for a warm-up + timed pass)"
     else:
         times = [one() for _ in range(iters)]
@@ -177,17 +180,39 @@ def run_reference(args, rank):
         return
     import torch
     from oracle import port
-    steps = max(1, min(args.steps, 3))
-    val, cores, sample = cpu_baseline(port, torch, args.frames, args.text_len, args.queries, iters=steps,
+    val, cores, sample = cpu_baseline(port, torch, args.frames, args.text_len, args.queries, iters=args.steps,
                                       warmup=1 if args.warmup > 0 else 0)
-    line = dict(metric=METRIC, value=val, unit="samples/s", n_gpus=args.gpus, steps=steps, warmup=1 if args.warmup > 0 else 0,
+    line = dict(metric=METRIC, value=val, unit="samples/s", n_gpus=args.gpus, steps=args.steps, warmup=1 if args.warmup > 0 else 0,
                 ms_per_step=1000.0 / val, higher_is_better=True, scaling="weak", vs_baseline=None, dtype="f32",
                 data="synthetic", impl="reference",
                 config=dict(workload="mPLUG-Video GPT-3 1.3B pretrain step, 8f x 224^2, text 128, 128 queries",
-                            per_step="1 sample fwd+bwd (bounded sample of the 32/GPU workload)", note=f"steps capped at {steps}"),
+                            per_step="1 sample fwd+bwd (bounded sample of the 32/GPU workload)"),
                 cpu_baseline=dict(value=val, unit="samples/s", cores=cores, kind="port", sample=sample),
                 e2e=dict(value=val, unit="samples/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0), gpu_launches=0)
     print(json.dumps(line), flush=True)
+
+
+DUMP_SAMPLE = 1 << 21     # values drawn from each flat training-state vector by --dump-outputs (8 MB each in fp32)
+
+
+def dump_outputs(out_dir, eng, loss):
+    """--dump-outputs: what the last timed step handed back, as float32 / float64 .npy files - its loss, the global
+    gradient norm AdamW clipped with, and, at a fixed seeded sample of DUMP_SAMPLE flat positions (sample_index.npy),
+    the trainable parameters it wrote (fp32 master copy) and AdamW's first moment.  With the same arguments the
+    inputs and initial weights are the same from run to run and every reduction of the step adds in a fixed order,
+    so one build writes the same bits every run and two builds can be compared file by file."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = eng.master.numel()
+    idx = torch.randint(0, n, (min(DUMP_SAMPLE, n),), generator=torch.Generator().manual_seed(0)).sort().values
+    arrays = dict(loss=np.asarray([float(loss.float().item())], dtype=np.float32),
+                  grad_norm=np.asarray([float(eng.optimizer._global_grad_norm)], dtype=np.float64),
+                  sample_index=idx.numpy().astype(np.float64),
+                  trainable_params=eng.master[idx.to(eng.master.device)].cpu().numpy(),
+                  adam_exp_avg=eng.exp_avg[idx.to(eng.exp_avg.device)].cpu().numpy())
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_ymp(args, rank, local_rank, world):
@@ -284,6 +309,8 @@ def run_ymp(args, rank, local_rank, world):
     if rank == 0:
         sampler.start()
     ms, last_loss = timed(step_resident, args.steps)
+    if args.dump_outputs and rank == 0:     # before any further step changes the weights
+        dump_outputs(args.dump_outputs, eng, last_loss)
     # kernels of ours enqueued per timed step: counted on one eager step (a graph replay re-launches the
     # same kernels without going through the library's host entry points)
     n0 = lib.launch_count()
@@ -420,7 +447,7 @@ def run_ymp(args, rank, local_rank, world):
         del eng, model
         torch.cuda.empty_cache()
         from oracle import port          # the CPU restatement, timed as the baseline only (never on the product path)
-        val, cores, sample = cpu_baseline(port, torch, T, L, Q, iters=3, warmup=1)
+        val, cores, sample = cpu_baseline(port, torch, T, L, Q, iters=3, warmup=1, cold_cutoff_s=90.0)
         line["cpu_baseline"] = dict(value=val, unit="samples/s", cores=cores, kind="port", sample=sample)
     print(json.dumps(line), flush=True)
     if world > 1:
@@ -469,7 +496,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--gemm-report", default=None, help="write per-shape GEMM timings of one step to this json file")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly (no CUDA graph replay)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the last one's loss, grad norm and a seeded sample of the updated "
+                         "trainable parameters and AdamW first moment to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ymp":
+        ap.error("--dump-outputs writes the results of the B200 path (--impl ymp)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -336,6 +336,33 @@ def run_hostside(name):
           f"({os.path.getsize(path) / 1024:.0f} KiB)", flush=True)
 
 
+def run_task_configs(name):
+    """Stores what the reference ships as data for its task scripts: every configs/**/*.yaml parsed with the YAML loader
+    the scripts use (the package's ruamel.yaml stand-in: 1e-6 is a float), keyed by its path under configs/, and the
+    class-name table of the classification task (classname.json).  tests/test_host_cpu.py compares the package's yamls
+    with the first; the downstream workspace of tests/plumbing.py takes its labels from the second."""
+    import glob
+    import importlib
+    import json
+    compat = os.path.join(ROOT, "youku-mplug_b200", "compat")
+    sys.path.append(compat)
+    try:
+        ryaml = importlib.import_module("ruamel.yaml")
+    finally:
+        sys.path.remove(compat)
+    cfg_root = os.path.join(ref_shims.REFERENCE_ROOT, "configs")
+    paths = sorted(glob.glob(os.path.join(cfg_root, "**", "*.yaml"), recursive=True))
+    configs = {os.path.relpath(p, cfg_root): ryaml.load(open(p), Loader=ryaml.Loader) for p in paths}
+    with open(os.path.join(ref_shims.REFERENCE_ROOT, "classname.json")) as f:
+        classnames = json.load(f)
+    path = os.path.join(GOLD, name + ".json")
+    with open(path, "w") as f:
+        json.dump(dict(configs=configs, classnames=classnames), f, indent=1)
+        f.write("\n")
+    print(f"[{name}] {len(configs)} task configs, {len(classnames)} class names; wrote {path} "
+          f"({os.path.getsize(path) / 1024:.0f} KiB)", flush=True)
+
+
 def run_generate(name, vcfg, gcfg, Q, B, L, wseed, iseed, beam_size=3, n_new=6, pos_gain=30.0, ln_gain=16.0, stop_after=3):
     """Golden vectors for the generation path (SURVEY 8f N2): the UNMODIFIED reference's per-sample beam
     search and batched greedy sampling over its KV cache, with the visual prefix, next to the oracle's
@@ -608,6 +635,7 @@ if __name__ == "__main__":
     ap.add_argument("--only-dropout", action="store_true", help="only (re)write the decoder-dropout fixture")
     ap.add_argument("--only-generate", action="store_true", help="only (re)write the generation fixture")
     ap.add_argument("--only-downstream", action="store_true", help="only (re)write the downstream-model fixture")
+    ap.add_argument("--only-task-configs", action="store_true", help="only (re)write the task-config / class-name fixture")
     a = ap.parse_args()
     torch.set_num_threads(os.cpu_count())
     if a.caption27b:
@@ -626,6 +654,10 @@ if __name__ == "__main__":
     if a.only_downstream:
         run_downstream("tiny_downstream", port.VCFG_TINY, port.GCFG_TINY, Q=8, wseed=21)
         sys.exit(0)
+    if a.only_task_configs:
+        run_task_configs("reference_task_configs")
+        sys.exit(0)
+    run_task_configs("reference_task_configs")
     run_hostside("tiny_hostside")
     run_image("tiny_pretrain_image", port.ECFG_TINY, port.GCFG_TINY, Q=8, B=2, L=8, wseed=71, iseed=72)
     run_generate("tiny_generate", port.VCFG_TINY, port.GCFG_TINY, Q=8, B=2, L=8, wseed=51, iseed=52)

@@ -98,7 +98,8 @@ def make_downstream_workspace(td, task, num_videos=8, batch_size=2, max_length=8
     words = "a b c d e f g hello world video cat dog runs on the grass".split()
     clips = [f"clip{i}.npy" for i in range(num_videos)]
     if task == "cls":
-        classes = list(json.load(open(os.path.join(os.environ.get("YMP_REFERENCE", "/root/reference"), "classname.json"))))
+        with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_task_configs.json")) as f:
+            classes = list(json.load(f)["classnames"])       # the reference's classname.json
         header, rows = "video_id:FILE,title,label", [f"{c},{' '.join(rng.choice(words, 3))},{classes[i % len(classes)]}" for i, c in enumerate(clips)]
         prefix, extra = "classification", "use_cls: true\nnum_frames: %d\nnum_classes: %d\n" % (num_frames, len(classes))
     elif task == "caption":

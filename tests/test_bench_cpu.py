@@ -37,6 +37,12 @@ def test_reference_arm_is_silent_on_other_ranks():
     assert r.returncode == 0 and r.stdout.strip() == "", (r.stdout, r.stderr[-500:])
 
 
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], cwd=ROOT, capture_output=True,
+                       text=True, timeout=600)
+    assert r.returncode != 0 and "--steps" in r.stderr and not r.stdout.strip()
+
+
 def test_product_arm_refuses_to_run_without_a_gpu():
     """No CPU fallback, no silent substitute number: without a CUDA device the product arm exits non-zero and prints no
     JSON line (the oracle is never on its path)."""

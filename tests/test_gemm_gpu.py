@@ -159,7 +159,7 @@ def test_gemm_pair_tile_tma_epilogue_variants(cuda, M):
     mul = torch.randn(M, K, device=cuda).bfloat16()
     g = ops.gemm(a.new_empty(M, N).normal_().bfloat16(), b, b_t=True, aux_in=mul, act=1, tile_n=512)
     assert g.shape == (M, K)
-    # split-K wgrad: fp32 accumulate (bulk reduce-add) into a running buffer
+    # split-K wgrad: fp32 accumulate into a running buffer (slices added in order by the reduction kernel)
     dy = torch.randn(M, N, device=cuda).bfloat16()
     acc = torch.full((N, K), 0.5, device=cuda)
     ops.gemm(dy, a, a_t=True, b_t=True, out=acc, accumulate=True, split_k=3, tile_n=512)

@@ -206,7 +206,6 @@ def test_task_configs_mirror_the_reference_yamls():
     """configs/{pretrain,caption,cls,retrieval}/*.yaml: every file the reference ships for the GPT-3 models exists here
     under the same name, parses with the YAML loader the scripts use (ruamel.yaml semantics: 1e-6 is a float), and
     carries the same keys and values as the reference's file except for megatron_cfg (tensor parallel size 1 here)."""
-    import glob
     import importlib
     import sys
     compat = os.path.join(ROOT, "youku-mplug_b200", "compat")
@@ -223,19 +222,19 @@ def test_task_configs_mirror_the_reference_yamls():
              "retrieval/retrieval_gpt3_1.3B_youku_v0.yaml", "retrieval/retrieval_gpt3_2.7B_youku_v0.yaml",
              "retrieval/retrieval_itm_gpt3_1.3B_youku_v0.yaml", "retrieval/retrieval_itm_gpt3_2.7B_youku_v0.yaml",
              "pretrain/gpt3_1.3B/pretrain_gpt3_freezeGPT_youku_v0.yaml", "pretrain/gpt3_2.7B/pretrain_gpt3_freezeGPT_youku_v0.yaml"]
-    ref_root = "/root/reference/configs"
+    # the reference's own yamls, parsed with the same loader (oracle/make_golden.py run_task_configs)
+    with open(os.path.join(ROOT, "tests", "golden", "reference_task_configs.json")) as f:
+        ref_configs = json.load(f)["configs"]
     for n in names:
         cfg = ryaml.load(open(os.path.join(cfg_root, n)), Loader=ryaml.Loader)
         assert cfg["megatron_cfg"]["tensor_model_parallel_size"] == 1 and cfg["megatron_cfg"]["model_parallel_size"] == 1
         assert isinstance(cfg["optimizer"]["lr"], float) and isinstance(cfg["optimizer"]["opt_eps"], float)
         assert isinstance(cfg["schedular"]["min_lr"], float) and cfg["freeze_text_decoder"] is True and cfg["num_learnable_token"] == 128
         assert os.path.exists(os.path.join(ROOT, "youku-mplug_b200", cfg["text_cfg"])) and os.path.exists(os.path.join(ROOT, "youku-mplug_b200", cfg["visual_cfg"]))
-        if os.path.isdir(ref_root):   # (the reference checkout exists in the development container only)
-            ref = ryaml.load(open(os.path.join(ref_root, n)), Loader=ryaml.Loader)
-            assert set(ref) == set(cfg), (n, set(ref) ^ set(cfg))
-            for k in ref:
-                if k != "megatron_cfg":
-                    assert ref[k] == cfg[k], (n, k, ref[k], cfg[k])
-    if os.path.isdir(ref_root):
-        shipped = {os.path.relpath(p, ref_root) for p in glob.glob(os.path.join(ref_root, "*", "*.yaml")) + glob.glob(os.path.join(ref_root, "pretrain", "*", "*.yaml"))}
-        assert shipped <= set(names) | {n for n in shipped if "b200" in n}, shipped - set(names)
+        ref = ref_configs[n]
+        assert set(ref) == set(cfg), (n, set(ref) ^ set(cfg))
+        for k in ref:
+            if k != "megatron_cfg":
+                assert ref[k] == cfg[k], (n, k, ref[k], cfg[k])
+    shipped = set(ref_configs)
+    assert shipped <= set(names) | {n for n in shipped if "b200" in n}, shipped - set(names)

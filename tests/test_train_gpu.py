@@ -78,7 +78,7 @@ def _batches(n, cuda, B=2, L=8):
 def test_graph_train_step_equals_eager_loop(cuda):
     """4 consecutive iterations: CUDA-graph replay (captured at the 2nd call) vs the reference loop's
     model(); model.backward(loss); model.step().  The weight-gradient accumulators are zeroed between
-    replays by step(); split-K / LayerNorm atomics make fp32 sums order-dependent, hence the tolerances."""
+    replays by step(); the comparisons keep a tolerance for fp32 rounding."""
     from ymp.train import TrainEngine
     lr = 1e-3
     eng_g = TrainEngine(_tiny(cuda), lr=lr)
@@ -155,7 +155,7 @@ def test_checkpoint_round_trip(cuda):
     # the module's parameters are views of flat_param: the model sees the restored weights
     p0 = next(p for p in eng.module.parameters() if p.requires_grad)
     assert p0.data_ptr() >= eng.flat_param.data_ptr() and p0.data_ptr() < eng.flat_param.data_ptr() + eng.flat_param.numel() * 2
-    # a fresh engine loading `latest` continues identically (up to atomics order)
+    # a fresh engine loading `latest` continues identically (up to fp32 rounding)
     eng2 = TrainEngine(_tiny(cuda, seed=99), lr=1e-3)
     eng2.load_checkpoint(td)
     loss2 = eng2.train_step(*batches[2], use_graph=False).item()

@@ -79,7 +79,7 @@ def ncu_shapes():
         ops.gemm(x, w3)                                        # GPT h->4h
     g = torch.zeros(768, 768, device=dev)
     for _ in range(2):
-        ops.gemm(dy[:50176], a, a_t=True, b_t=True, out=g, accumulate=True)   # wgrad, split-K atomics
+        ops.gemm(dy[:50176], a, a_t=True, b_t=True, out=g, accumulate=True)   # wgrad, split-K
     torch.cuda.synchronize()
 
 

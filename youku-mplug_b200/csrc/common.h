@@ -83,4 +83,22 @@ struct DeviceMax {
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// Deterministic reductions.  A kernel whose blocks (or split-K slices) each produce a partial sum of the same outputs
+// writes the partials to scratch memory instead of adding them with atomics, whose order depends on scheduling; a
+// second kernel then adds the partials in an order fixed by the shapes alone, so a run gives the same bits every time.
+// The scratch is stream-ordered (cudaMallocFromPoolAsync / cudaFreeAsync on the caller's stream, from a memory pool
+// of the library's own that keeps freed blocks for the next call), which also holds inside CUDA-graph capture, where
+// it becomes a graph allocation node.  A Scratch gives its block back when it goes out of scope, so every return path,
+// error returns included, frees it; release() frees it early and reports the status.
+struct Scratch {
+  void* p = nullptr;
+  cudaStream_t st = nullptr;
+  int alloc(size_t bytes, cudaStream_t stream);
+  int release();
+  ~Scratch() { if (p) cudaFreeAsync(p, st); }
+};
+// out[c] += sum over b = 0 .. nblk-1 of part[b * ldp + c], c < C (fp32); with out2, columns c >= C1 go to out2[c - C1]
+int reduce_partials(const float* part, int nblk, long ldp, int C, float* out, cudaStream_t st, float* out2 = nullptr,
+                    int C1 = 0);
+
 }  // namespace ymp

@@ -2,9 +2,10 @@
 //   warp 0      : TMA producer   (cp.async.bulk.tensor 2D, SWIZZLE_128B, NSTAGE-deep mbarrier ring)
 //   warp 1      : MMA issuer     (tcgen05.mma cta_group::1 kind::f16, 128 x BN x 16, fp32 accum in TMEM)
 //   warp 2      : TMEM allocator (2 accumulator stages so the epilogue of tile i overlaps tile i+1)
-//   warps 4..11 : epilogue       (tcgen05.ld -> bias / GELU / GELU' / residual -> bf16|fp32|atomic fp32)
+//   warps 4..11 : epilogue       (tcgen05.ld -> bias / GELU / GELU' / residual -> bf16|fp32|fp32 accumulate)
 // Operands may be K-major or MN-major (both handled by the UMMA smem descriptors), so the same
-// kernel serves forward (x.W^T), dgrad (dy.W) and wgrad (dy^T.x, split-K with fp32 atomics).
+// kernel serves forward (x.W^T), dgrad (dy.W) and wgrad (dy^T.x, split-K slices
+// reduced in a fixed order, see ymp_gemm).
 #include <cuda.h>
 
 #include "common.h"
@@ -41,7 +42,8 @@ struct GemmKParams {
   DropSpec drop;                   // dropout before the residual add (has_drop)
   int has_drop;
   int epi_tma;                     // CTA-pair kernel: outputs staged in swizzled smem and written by TMA (bulk tensor
-                                   // store; bulk reduce-add for the fp32 split-K accumulation)
+                                   // store; bulk reduce-add for the fp32 accumulation; one K slice only)
+  long long d_split_stride;        // split-K: slice ks of the K range writes D + ks * d_split_stride (0: no split)
 };
 
 template <int BN>
@@ -146,7 +148,7 @@ __device__ __forceinline__ void epilogue_prefetch(const GemmKParams& p, int row,
 // Epilogue for one thread: 32 consecutive columns of one output row.
 template <bool DROP>
 __device__ __forceinline__ void epilogue_chunk(const GemmKParams& p, const uint32_t (&r)[32],
-                                               int row, int col0, const EpiPrefetch& pf, const DropState& ds) {
+                                               int row, int col0, const EpiPrefetch& pf, const DropState& ds, size_t dsplit) {
   if (row >= p.M || col0 >= p.N) return;
   const bool full = (col0 + 32 <= p.N);
   const int drow = p.d_row_block ? (row / p.d_row_block) * p.d_row_stride + row % p.d_row_block : row;
@@ -166,7 +168,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmKParams& p, const uint3
       for (int i = 0; i < 16; ++i) { v[2 * i] += bf16_lo(pf.bias[i]); v[2 * i + 1] += bf16_hi(pf.bias[i]); }
     }
     const size_t off = (size_t)row * p.ldd + col0;          // aux tensors: plain rows
-    const size_t doff = (size_t)drow * p.ldd + col0;        // D: optionally re-blocked rows
+    const size_t doff = dsplit + (size_t)drow * p.ldd + col0;   // D: optionally re-blocked rows
     // aux_out: with an activation it receives act'(v) (what the backward epilogue multiplies by),
     // without one the value itself.  aux_in: a plain multiplier.  Switches are warp-uniform.
     if (p.aux_in) {
@@ -261,7 +263,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmKParams& p, const uint3
       if (col < p.N) {
         float x = v[i];
         if (p.bias) x += __bfloat162float(p.bias[col]);
-        const size_t off = (size_t)row * p.ldd + col, doff = (size_t)drow * p.ldd + col;
+        const size_t off = (size_t)row * p.ldd + col, doff = dsplit + (size_t)drow * p.ldd + col;
         if (p.aux_in) {
           x *= __bfloat162float(p.aux_in[off]);
         } else if (p.act == YMP_ACT_GELU_ERF) {
@@ -614,7 +616,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a,
           __syncwarp();
           if (lane == 0) mbar_arrive(&tempty_bar[as]);
         }
-        epilogue_chunk<DROP>(p, r, row, n_blk * BN + coff, pf, ds);
+        epilogue_chunk<DROP>(p, r, row, n_blk * BN + coff, pf, ds, (size_t)(u % p.split_k) * p.d_split_stride);
       }
       if (++as == 2) { as = 0; aphase ^= 1; }
     }
@@ -910,7 +912,7 @@ gemm_bf16_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tma_a,
           __syncwarp();
           if (lane == 0) mbar_arrive_cluster(&tempty_bar[as], 0);  // always on the leader's barrier
         }
-        epilogue_chunk<DROP>(p, r, row, n_blk * BN2 + coff, pf, ds);
+        epilogue_chunk<DROP>(p, r, row, n_blk * BN2 + coff, pf, ds, (size_t)(u % p.split_k) * p.d_split_stride);
       }
       }
 #ifdef YMP_GEMM_DBG
@@ -1003,6 +1005,37 @@ static int make_out_map(CUtensorMap* m, const void* ptr, bool f32, uint64_t inne
   return YMP_OK;
 }
 
+// Split-K: D[r, c] += ws[0][r, c] + ws[1][r, c] + ... + ws[split-1][r, c], slices added in order (deterministic).
+// Blocks (x, y) take rows y, y + gridDim.y, ...; 4 consecutive columns per thread (ldw, ldd are multiples of 8 and both
+// bases 16-byte aligned).  D rows follow the GEMM's optional re-blocking (d_row_block / d_row_stride).
+__global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restrict__ ws, int split, long long slice, int M,
+                                                            int N, int ldw, float* __restrict__ D, int ldd, int d_row_block,
+                                                            int d_row_stride) {
+  const int c = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+  if (c >= N) return;
+  for (int r = blockIdx.y; r < M; r += gridDim.y) {
+    const int drow = d_row_block ? (r / d_row_block) * d_row_stride + r % d_row_block : r;
+    const float* w = ws + (size_t)r * ldw + c;
+    float* d = D + (size_t)drow * ldd + c;
+    if (c + 4 <= N) {
+      float4 s = *reinterpret_cast<const float4*>(w);
+      for (int k = 1; k < split; ++k) {
+        const float4 x = *reinterpret_cast<const float4*>(w + (size_t)k * slice);
+        s.x += x.x; s.y += x.y; s.z += x.z; s.w += x.w;
+      }
+      float4 o = *reinterpret_cast<float4*>(d);
+      o.x += s.x; o.y += s.y; o.z += s.z; o.w += s.w;
+      *reinterpret_cast<float4*>(d) = o;
+    } else {
+      for (int e = 0; c + e < N; ++e) {
+        float s = w[e];
+        for (int k = 1; k < split; ++k) s += w[(size_t)k * slice + e];
+        d[e] += s;
+      }
+    }
+  }
+}
+
 template <int BN>
 static int launch_gemm(const ymp_gemm_args* a, const GemmKParams& kp, cudaStream_t stream) {
   using Cfg = GemmCfg<BN>;
@@ -1042,7 +1075,7 @@ static int launch_gemm_2cta(const ymp_gemm_args* a, GemmKParams kp, cudaStream_t
   static const bool no_tma_epi = [] { const char* e = getenv("YMP_GEMM_LEGACY_EPI"); return e && e[0] == '1'; }();
   static const int tma_epi_max_k = [] { const char* e = getenv("YMP_GEMM_TMA_EPI_MAXK"); return e ? atoi(e) : 1024; }();
   const bool f32 = a->out_dtype == YMP_DT_F32;
-  kp.epi_tma = (!no_tma_epi && a->K <= tma_epi_max_k && a->N % 64 == 0 && a->d_row_block == 0 && (a->ldd * (f32 ? 4 : 2)) % 16 == 0 &&
+  kp.epi_tma = (!no_tma_epi && kp.split_k == 1 && a->K <= tma_epi_max_k && a->N % 64 == 0 && a->d_row_block == 0 && (a->ldd * (f32 ? 4 : 2)) % 16 == 0 &&
                 !(f32 && a->aux_out)) ? 1 : 0;
   if (kp.epi_tma) {
     rc = make_out_map(&td, a->D, f32, a->N, a->M, a->ldd);
@@ -1138,9 +1171,11 @@ extern "C" int ymp_gemm(const ymp_gemm_args* a, void* stream) {
     if (a->accumulate) {
       const long tiles = bn == 512 ? (long)((a->M + 2 * BM - 1) / (2 * BM)) * ((a->N + 255) / 256)
                                    : (long)((a->M + BM - 1) / BM) * ((a->N + bn - 1) / bn);
-      // cost model (k-blocks of MMA time): waves x (k-blocks per unit + a fixed pipeline-fill / atomic-epilogue
-      // overhead of ~24 k-blocks).  Measured on the ViT wgrads: 768x768x50208 is fastest at 8 splits
-      // (72 units = one wave of the 74 CTA pairs, 53 us vs 82 us at 32 splits), 3072x768 at 2.
+      // cost model (k-blocks of MMA time): waves x (k-blocks per unit + a fixed pipeline-fill / split-epilogue
+      // overhead of ~24 k-blocks).  Tuned on the ViT wgrads when the slices were added with atomics:
+      // 768x768x50208 was fastest at 8 splits (72 units = one wave of the 74 CTA pairs, 53 us vs 82 us at 32
+      // splits), 3072x768 at 2.  With the ordered reduction through scratch, 768x768x50432 takes 46.3 us (GEMM) + 4.4 us
+      // (reduction) against 49.1 us with atomics (torch.profiler, B200 at 1000 W); the split counts were not re-tuned.
       const long workers = bn == 512 ? sms / 2 : sms;
       long best = -1;
       for (int sp = 1; sp <= 64 && sp * 8 <= kb_total; ++sp) {
@@ -1183,10 +1218,32 @@ extern "C" int ymp_gemm(const ymp_gemm_args* a, void* stream) {
   kp.v32_aux = (a->ldd * 2) % 32 == 0 && (!a->aux_out || al32(a->aux_out)) && (!a->aux_in || al32(a->aux_in));
   kp.v32_res = a->residual && al32(a->residual) && (a->ldr * 2) % 32 == 0;
   kp.v32_bias = a->bias && al32(a->bias);
+  kp.d_split_stride = 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (bn == 512) return launch_gemm_2cta(a, kp, st);
-  if (bn == 256) return launch_gemm<256>(a, kp, st);
-  return launch_gemm<128>(a, kp, st);
+  if (split == 1) {
+    if (bn == 512) return launch_gemm_2cta(a, kp, st);
+    if (bn == 256) return launch_gemm<256>(a, kp, st);
+    return launch_gemm<128>(a, kp, st);
+  }
+  // split-K: every slice stores its partial product to its own fp32 scratch matrix (no atomics), then
+  // splitk_reduce_kernel adds the slices into D in slice order, so the result does not depend on scheduling
+  // (the scratch rows are plain: the reduction applies D's row re-blocking)
+  const int ldw = (a->N + 7) / 8 * 8;
+  Scratch ws;
+  int rc = ws.alloc(sizeof(float) * (size_t)split * a->M * ldw, st);
+  if (rc) return rc;
+  kp.D = ws.p; kp.ldd = ldw; kp.accumulate = 0;
+  kp.d_row_block = 0; kp.d_row_stride = 0;
+  kp.d_split_stride = (long long)a->M * ldw;
+  kp.v32_d = al32(ws.p) && (ldw * 4) % 32 == 0;
+  rc = bn == 512 ? launch_gemm_2cta(a, kp, st) : bn == 256 ? launch_gemm<256>(a, kp, st) : launch_gemm<128>(a, kp, st);
+  if (rc) return rc;
+  const int vec = (a->N + 3) / 4;
+  const int tpb = vec < 256 ? (vec + 31) / 32 * 32 : 256;
+  splitk_reduce_kernel<<<dim3((vec + tpb - 1) / tpb, a->M < 65535 ? a->M : 65535), tpb, 0, st>>>(
+      (const float*)ws.p, split, kp.d_split_stride, a->M, a->N, ldw, (float*)a->D, a->ldd, a->d_row_block, a->d_row_stride);
+  YMP_LAUNCH_CHECK();
+  return ws.release();
 }
 
 #ifdef YMP_GEMM_DBG

@@ -122,8 +122,9 @@ struct LnBwdParams {
   const float* rstd;
   const __nv_bfloat16* add;  // optional gradient of the residual branch, added to dx
   __nv_bfloat16* dx;
-  float* dgamma;  // fp32 [D], accumulated with atomics (caller zeroes); NULL = frozen
+  float* dgamma;  // fp32 [D], accumulated (caller zeroes); NULL = frozen
   float* dbeta;
+  float* wpart;   // with dgamma: per-block partials, row b = [dgamma part (D) | dbeta part (D)], added by reduce_partials
   const int32_t* in_rows;
   int rows, D, ldx, lddy, ldadd;
   __nv_bfloat16* dx_drop;  // optional: dx with the dropout mask of the site that produced x applied
@@ -200,7 +201,7 @@ __global__ void __launch_bounds__(LN_WARPS * 32, WGRAD ? (VPL <= 4 ? 3 : 1) : (D
     }
   }
   if (WGRAD) {
-    // block-level reduce across the 8 warps, then one atomic per column per block
+    // block-level reduce across the 8 warps, then this block's partials go to its row of p.wpart
     __shared__ float red[LN_WARPS][32 * 8 + 1];
     for (int j = 0; j < VPL; ++j) {
       for (int pass = 0; pass < 2; ++pass) {
@@ -216,12 +217,12 @@ __global__ void __launch_bounds__(LN_WARPS * 32, WGRAD ? (VPL <= 4 ? 3 : 1) : (D
 #pragma unroll
             for (int e = 0; e < 4; ++e) s[e] += red[w][threadIdx.x * 4 + e];
           const int col = j * 256 + threadIdx.x * 4;
-          float* dst = (pass == 0 ? p.dgamma : p.dbeta) + col;
+          float* dst = p.wpart + (size_t)blockIdx.x * 2 * p.D + pass * p.D + col;
           if (col + 3 < p.D) {
-            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(s[0]), "f"(s[1]), "f"(s[2]), "f"(s[3]) : "memory");
+            *reinterpret_cast<float4*>(dst) = make_float4(s[0], s[1], s[2], s[3]);
           } else {
             for (int e = 0; e < 4; ++e)
-              if (col + e < p.D) atomicAdd(dst + e, s[e]);
+              if (col + e < p.D) dst[e] = s[e];
           }
         }
       }
@@ -278,8 +279,6 @@ extern "C" int ymp_layernorm_bwd(const ymp_layernorm_bwd_args* a, void* stream) 
   cudaStream_t st = (cudaStream_t)stream;
   const int vpl = (a->D / 8 + 31) / 32;
   const bool wg = a->dgamma != nullptr;
-  // with weight grads each block ends with 2*D atomics; 6 blocks per SM keeps enough warps in
-  // flight for HBM while bounding the atomic tail (~900 adds per address)
   // resident blocks per SM: 3 with weight grads (80 registers at D <= 1024), 4 without; the grid is a whole
   // number of such waves so that the row loop stays balanced
   const int cap = wg ? num_sms() * (a->D <= 1024 ? 3 : 2) : num_sms() * 8;
@@ -288,10 +287,20 @@ extern "C" int ymp_layernorm_bwd(const ymp_layernorm_bwd_args* a, void* stream) 
   const bool xf = (a->x_dtype == YMP_DT_F32);
 #define YMP_LN_BWD(V, W, X) do { if (p.dx_drop) ln_bwd_kernel<V, W, X, true><<<blocks, thr, 0, st>>>(p); else ln_bwd_kernel<V, W, X, false><<<blocks, thr, 0, st>>>(p); } while (0)
 #define YMP_LN_BWD_V(W, X) do { if (vpl <= 3) YMP_LN_BWD(3, W, X); else if (vpl <= 8) YMP_LN_BWD(8, W, X); else YMP_LN_BWD(16, W, X); } while (0)
+  Scratch part;
+  p.wpart = nullptr;
+  if (wg) {
+    const int rc = part.alloc(sizeof(float) * 2 * (size_t)a->D * blocks, st);
+    if (rc) return rc;
+    p.wpart = (float*)part.p;
+  }
   if (wg) { if (xf) YMP_LN_BWD_V(true, true); else YMP_LN_BWD_V(true, false); }
   else { if (xf) YMP_LN_BWD_V(false, true); else YMP_LN_BWD_V(false, false); }
 #undef YMP_LN_BWD_V
 #undef YMP_LN_BWD
   YMP_LAUNCH_CHECK();
-  return YMP_OK;
+  if (!wg) return YMP_OK;
+  const int rc = reduce_partials(p.wpart, blocks, 2L * a->D, 2 * a->D, a->dgamma, st, a->dbeta, a->D);
+  if (rc) return rc;
+  return part.release();
 }

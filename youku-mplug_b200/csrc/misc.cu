@@ -194,15 +194,15 @@ __global__ void __launch_bounds__(CE_THREADS) ce_bwd_kernel(const __nv_bfloat16*
 // out[c] += sum_r in[r, c]   (fp32; the caller zeroes or carries `out`).
 // Block = 8 warps x 32 lanes: a warp reads 512 contiguous bytes of one row (8 columns per lane, 8 rows
 // in flight per lane), the 8 warps of a block take interleaved rows and are reduced through shared
-// memory, so a block issues ONE 16-byte vector reduction per 4 columns: same-address atomic traffic
-// (the limiter of the first version at C=768) drops by 32x.
+// memory; block (x, y) writes its partial column sums to row y of `part` (ldp floats per row), and reduce_partials
+// adds the rows in order.
 constexpr int CS_WARPS = 8;
 __device__ __forceinline__ void acc8(float (&acc)[8], const uint4& u) {
   acc[0] += bf16_lo(u.x); acc[1] += bf16_hi(u.x); acc[2] += bf16_lo(u.y); acc[3] += bf16_hi(u.y);
   acc[4] += bf16_lo(u.z); acc[5] += bf16_hi(u.z); acc[6] += bf16_lo(u.w); acc[7] += bf16_hi(u.w);
 }
 __global__ void __launch_bounds__(CS_WARPS * 32) colsum_kernel(const __nv_bfloat16* __restrict__ in,
-                                                               float* __restrict__ out, int R, int C, int ld,
+                                                               float* __restrict__ part, int ldp, int R, int C, int ld,
                                                                int rows_per_block) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int v = blockIdx.x * 32 + lane;  // 8-column vector index
@@ -234,11 +234,12 @@ __global__ void __launch_bounds__(CS_WARPS * 32) colsum_kernel(const __nv_bfloat
 #pragma unroll
       for (int e = 0; e < 4; ++e) s[e] += red[w][l][e0 + e];
     const int col = (blockIdx.x * 32 + l) * 8 + e0;
+    float* dst = part + (size_t)blockIdx.y * ldp + col;
     if (col + 3 < C) {
-      asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(out + col), "f"(s[0]), "f"(s[1]), "f"(s[2]), "f"(s[3]) : "memory");
+      *reinterpret_cast<float4*>(dst) = make_float4(s[0], s[1], s[2], s[3]);
     } else {
       for (int e = 0; e < 4; ++e)
-        if (col + e < C) atomicAdd(out + col + e, s[e]);
+        if (col + e < C) dst[e] = s[e];
     }
   }
 }
@@ -447,9 +448,16 @@ extern "C" int ymp_colsum(const ymp_colsum_args* a, void* stream) {
   int splits = max(1, min((a->R + 63) / 64, (num_sms() * 4 + gx - 1) / gx));
   const int rpb = (a->R + splits - 1) / splits;
   splits = (a->R + rpb - 1) / rpb;
-  colsum_kernel<<<dim3(gx, splits), CS_WARPS * 32, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)a->in, a->out, a->R, a->C, a->ld, rpb);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int ldp = (a->C + 3) / 4 * 4;
+  Scratch part;
+  int rc = part.alloc(sizeof(float) * (size_t)splits * ldp, st);
+  if (rc) return rc;
+  colsum_kernel<<<dim3(gx, splits), CS_WARPS * 32, 0, st>>>((const __nv_bfloat16*)a->in, (float*)part.p, ldp, a->R, a->C, a->ld, rpb);
   YMP_LAUNCH_CHECK();
-  return YMP_OK;
+  rc = reduce_partials((const float*)part.p, splits, ldp, a->C, a->out, st);
+  if (rc) return rc;
+  return part.release();
 }
 
 extern "C" int ymp_group_reduce(const ymp_group_args* a, void* stream) {

@@ -6,7 +6,8 @@
 
 namespace ymp {
 
-__global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, long n, float* __restrict__ out) {
+// one partial sum per block (part[blockIdx.x]); reduce_partials adds them in block order
+__global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, long n, float* __restrict__ part) {
   float acc = 0.f;
   const long n4 = n >> 2;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
@@ -23,7 +24,7 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g,
     float v = s[threadIdx.x];
 #pragma unroll
     for (int o = 4; o > 0; o >>= 1) v += __shfl_xor_sync(0xffu, v, o);
-    if (threadIdx.x == 0) atomicAdd(out, v);
+    if (threadIdx.x == 0) part[blockIdx.x] = v;
   }
 }
 
@@ -92,9 +93,15 @@ extern "C" int ymp_sumsq(const float* g, int64_t n, float* out, void* stream) {
   YMP_CHECK_ARG(g && out && n > 0, "ymp_sumsq: bad args");
   YMP_CHECK_ARG(aligned16(g), "ymp_sumsq: g must be 16-byte aligned");
   const int blocks = (int)min((long)((n / 4 + 255) / 256) + 1, (long)num_sms() * 8);
-  sumsq_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(g, (long)n, out);
+  cudaStream_t st = (cudaStream_t)stream;
+  Scratch part;
+  int rc = part.alloc(sizeof(float) * blocks, st);
+  if (rc) return rc;
+  sumsq_kernel<<<blocks, 256, 0, st>>>(g, (long)n, (float*)part.p);
   YMP_LAUNCH_CHECK();
-  return YMP_OK;
+  rc = reduce_partials((const float*)part.p, blocks, 1, 1, out, st);
+  if (rc) return rc;
+  return part.release();
 }
 
 extern "C" int ymp_adamw(const ymp_adamw_args* a, void* stream) {

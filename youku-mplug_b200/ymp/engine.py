@@ -1,7 +1,7 @@
 """Hand-scheduled forward/backward of the mPLUG-Video pre-training hot path on the C-ABI kernels.
 
 No autograd inside: every stage saves exactly what its backward needs, weight gradients are
-accumulated in fp32 (split-K atomics in the GEMM epilogue), and the frozen GPT-3 decoder runs
+accumulated in fp32 (split-K slices added in a fixed order after the GEMM), and the frozen GPT-3 decoder runs
 dgrad only (SURVEY.md section 2.2: no wgrad GEMMs, no saved GEMM inputs).
 
 Weights are addressed by the reference's own state_dict keys.  `W` maps key -> bf16 CUDA tensor,
