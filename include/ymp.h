@@ -133,7 +133,10 @@ int ymp_gemm(const ymp_gemm_args* a, void* stream);
 
 /* Skinny GEMM for single-token decoding (KV-cache steps of sample() / beam_search(),
  * models/modeling_distributed_gpt3.py:1620-1886): y[M, N] = epilogue(x[M, K] . w[N, K]^T), 1 <= M <= 8.  One pass over the
- * weights, HBM-bound, no tensor cores (csrc/gemv.cu).  Epilogue: + bias[n], act (YMP_ACT_*), + residual[m, n], store. */
+ * weights, HBM-bound, mma.sync fed straight from global memory (csrc/gemv.cu).  Epilogue: + bias[n], act (YMP_ACT_*),
+ * + residual[m, n], store.  ymp_gemm_skinny_batch takes the same arguments with 1 <= M <= 64 (the step of a batch of beam
+ * searches: n_samples x beam rows); both compute row m of y from row m of x only, bit for bit, whatever M is (the kernel
+ * layout is chosen from N and K), so the two agree on every row. */
 typedef struct ymp_gemm_skinny_args {
   const void* x;         /* bf16 [M, K], row stride ldx */
   const void* w;         /* bf16 [N, K], row stride ldw (an nn.Linear weight) */
@@ -149,7 +152,7 @@ typedef struct ymp_gemm_skinny_args {
   int64_t ldy2, y2_off_stride;
   /* optional fused LayerNorm of the complete fp32 result (the next sub-layer's input): the CTA that finishes last
    * (ticket in *ln_counter, which must be 0 at launch and is reset to 0) writes ln_out[m, :] = LN(y[m, :]) in bf16 with
-   * exactly the arithmetic of ymp_layernorm_fwd - one kernel boundary less per sub-layer of the decoding step */
+   * exactly the arithmetic of ymp_layernorm_fwd - one kernel boundary less per sub-layer of the decoding step.  M <= 8 only. */
   const void* ln_gamma;  /* bf16 [N] */
   const void* ln_beta;   /* bf16 [N] */
   void* ln_out;          /* bf16 [M, N], row stride ld_ln */
@@ -158,6 +161,7 @@ typedef struct ymp_gemm_skinny_args {
   float ln_eps;
 } ymp_gemm_skinny_args;
 int ymp_gemm_skinny(const ymp_gemm_skinny_args* a, void* stream);
+int ymp_gemm_skinny_batch(const ymp_gemm_skinny_args* a, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * LayerNorm (fp32 statistics, bf16 in/out), one warp per row.
@@ -255,6 +259,11 @@ typedef struct ymp_attn_args {
   const int32_t* s_kv_dev; /* optional DEVICE scalar: only the first min(s_kv, *s_kv_dev) keys exist.  Lets a captured
                              CUDA graph of the single-token decoding step follow the growing KV cache (forward only,
                              served by the mma.sync kernels) */
+  const int32_t* kv_rows;  /* optional DEVICE table [n_seq, ld_kv_rows] (single-query decoding only, s_q == 1): key j of
+                             sequence s is row kv_rows[s * ld_kv_rows + j] of the k and v buffers (map_kv unused).  A beam
+                             reorder of a batched beam search then moves table entries, not cached keys; every entry
+                             below s_kv must be a valid row even past *s_kv_dev */
+  int32_t ld_kv_rows;
 } ymp_attn_args;
 int ymp_attn_fwd(const ymp_attn_args* a, void* stream);
 

@@ -10,6 +10,8 @@ import torch  # noqa: E402
 from ymp import lib, ops  # noqa: E402
 
 dev, bf16, rows = torch.device("cuda"), torch.bfloat16, int(os.environ.get("ROWS", "5"))
+# up to 8 rows: ymp_gemm_skinny (one beam search); 9-64 rows: ymp_gemm_skinny_batch (a batch of beam searches)
+skinny = ops.gemm_skinny if rows <= ops.SKINNY_MAX_ROWS else ops.gemm_skinny_batch
 for name, N, K, kw in (("qkv", 6144, 2048, {}), ("dense", 2048, 2048, dict(res=True)), ("fc1", 8192, 2048, dict(act=2)),
                        ("fc2", 2048, 8192, dict(res=True)), ("lm_head", 51200, 2048, dict(f32=True))):
     copies = max(4, int(600e6 // (N * K * 2)))
@@ -20,13 +22,13 @@ for name, N, K, kw in (("qkv", 6144, 2048, {}), ("dense", 2048, 2048, dict(res=T
     od = torch.float32 if (kw.get("res") or kw.get("f32")) else bf16
     out = torch.empty(rows, N, device=dev, dtype=od)
     for w in ws[:2]:
-        ops.gemm_skinny(x, w, bias=b, residual=r, act=kw.get("act", 0), out=out)
+        skinny(x, w, bias=b, residual=r, act=kw.get("act", 0), out=out)
     torch.cuda.synchronize()
     g = torch.cuda.CUDAGraph()
     lib.set_pdl(os.environ.get("PDL", "0") == "1")
     with torch.cuda.graph(g):
         for w in ws:
-            ops.gemm_skinny(x, w, bias=b, residual=r, act=kw.get("act", 0), out=out)
+            skinny(x, w, bias=b, residual=r, act=kw.get("act", 0), out=out)
     lib.set_pdl(0)
     g.replay()
     torch.cuda.synchronize()
@@ -38,6 +40,6 @@ for name, N, K, kw in (("qkv", 6144, 2048, {}), ("dense", 2048, 2048, dict(res=T
     e1.record()
     torch.cuda.synchronize()
     us = e0.elapsed_time(e1) / (reps * copies) * 1e3
-    print("SKINNY " + json.dumps(dict(shape=name, N=N, K=K, rows=rows, us=round(us, 2), gbs=round(N * K * 2 / us / 1e3, 1),
+    print("SKINNY " + json.dumps(dict(shape=name, N=N, K=K, rows=rows, entry=skinny.__name__, us=round(us, 2), gbs=round(N * K * 2 / us / 1e3, 1),
                                       unroll=os.environ.get("YMP_SKINNY_UNROLL", "4"), pdl=os.environ.get("PDL", "0"), ksplit=os.environ.get("YMP_SKINNY_KSPLIT", "auto"))))
     del ws, g

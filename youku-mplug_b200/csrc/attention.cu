@@ -116,6 +116,8 @@ struct AttnKParams {
   int lddo, hsdo, lddq, lddk, lddv, hsdq, hsdk, hsdv;
   SeqMap mdo, mdq, mdkv;
   const int* skv_dev;  // optional device scalar: number of keys that exist (KV-cache decoding under a CUDA graph)
+  const int* kv_rows;  // optional device table: key j of sequence s is K/V row kv_rows[s * ld_kv_rows + j] (decode kernel only)
+  int ld_kv_rows;
 };
 
 // effective lengths of sequence s (short last sequence when total_rows is set)
@@ -681,7 +683,9 @@ __global__ void __launch_bounds__(128) attn_bwd_dkdv_kernel(const AttnKParams p)
 // running maximum, and the 128 private rows meet once at the end through shared memory.  Nothing waits on a tile:
 // one round trip to the cache per 128 keys instead of a load / mma.sync / softmax pipeline on a 64-row tile with a
 // single live row.  Algorithmic bytes: 2 * s_kv * D * 2 per (sequence, head).
-template <int D>
+// TAB: keys are found through the per-sequence row table kv_rows (batched beam search: a beam reorder rewrites table
+// entries, never cached rows); the arithmetic is that of the map_kv variant, key for key.
+template <int D, bool TAB>
 __global__ void __launch_bounds__(128) attn_decode_kernel(const AttnKParams p) {
   constexpr int CH = D / 8;
   extern __shared__ __align__(16) uint8_t smem_attn[];
@@ -695,17 +699,20 @@ __global__ void __launch_bounds__(128) attn_decode_kernel(const AttnKParams p) {
   const RSeq mkv = resolve(p.mkv, s);
   const RMat Mk = rmat(p.k, mkv, p.ldk, h * p.hsk), Mv = rmat(p.v, mkv, p.ldv, h * p.hsv);
   const __nv_bfloat16* qrow = p.q + rrow(resolve(p.mq, s), 0) * p.ldq + h * p.hsq;
+  const int* tab = TAB ? p.kv_rows + (long)s * p.ld_kv_rows : nullptr;
+  const __nv_bfloat16* kbase = p.k + h * p.hsk;
+  const __nv_bfloat16* vbase = p.v + h * p.hsv;
   constexpr bool TWO_PHASE = D > 80;   // wide heads: V is requested after K has been consumed (register budget)
   uint4 qv[CH], kv[CH], vv[CH];
 #pragma unroll
   for (int c = 0; c < CH; ++c) qv[c] = __ldg(reinterpret_cast<const uint4*>(qrow) + c);
   auto fetch_k = [&](int key) {
-    const uint4* kr = reinterpret_cast<const uint4*>(mrow(Mk, key));
+    const uint4* kr = reinterpret_cast<const uint4*>(TAB ? kbase + (long)__ldg(tab + key) * p.ldk : mrow(Mk, key));
 #pragma unroll
     for (int c = 0; c < CH; ++c) kv[c] = __ldg(kr + c);
   };
   auto fetch_v = [&](int key) {
-    const uint4* vr = reinterpret_cast<const uint4*>(mrow(Mv, key));
+    const uint4* vr = reinterpret_cast<const uint4*>(TAB ? vbase + (long)__ldg(tab + key) * p.ldv : mrow(Mv, key));
 #pragma unroll
     for (int c = 0; c < CH; ++c) vv[c] = __ldg(vr + c);
   };
@@ -779,14 +786,18 @@ __global__ void __launch_bounds__(128) attn_decode_kernel(const AttnKParams p) {
   }
   if (p.lse && threadIdx.x == 0) p.lse[((long)s * p.n_heads + h) * p.s_q] = (m_all + log2f(l_all)) * 0.6931471805599453f;
 }
-template <int D>
-static int launch_decode(const AttnKParams& p, cudaStream_t st) {
+template <int D, bool TAB>
+static int launch_decode_t(const AttnKParams& p, cudaStream_t st) {
   constexpr int smem = (128 * (D + 1) + 128 + 4) * 4;
   static DeviceOnce once;
-  if (once.first()) { YMP_CUDA(cudaFuncSetAttribute(attn_decode_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); }
-  launch_k(attn_decode_kernel<D>, dim3(p.n_heads, p.n_seq), dim3(128), smem, st, p);
+  if (once.first()) { YMP_CUDA(cudaFuncSetAttribute(attn_decode_kernel<D, TAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); }
+  launch_k(attn_decode_kernel<D, TAB>, dim3(p.n_heads, p.n_seq), dim3(128), smem, st, p);
   YMP_LAUNCH_CHECK();
   return YMP_OK;
+}
+template <int D>
+static int launch_decode(const AttnKParams& p, cudaStream_t st) {
+  return p.kv_rows ? launch_decode_t<D, true>(p, st) : launch_decode_t<D, false>(p, st);
 }
 
 static int fill_params(const ymp_attn_args* a, AttnKParams& p, const char* who) {
@@ -811,6 +822,7 @@ static int fill_params(const ymp_attn_args* a, AttnKParams& p, const char* who) 
   p.mask = a->mask; p.mask_block = a->mask_block > 0 ? a->mask_block : 1; p.total_rows = a->total_rows;
   p.scale = a->scale; p.scale_log2 = a->scale * 1.4426950408889634f;
   p.skv_dev = a->s_kv_dev;
+  p.kv_rows = a->kv_rows; p.ld_kv_rows = a->ld_kv_rows;
   return YMP_OK;
 }
 
@@ -862,7 +874,11 @@ extern "C" int ymp_attn_fwd(const ymp_attn_args* a, void* stream) {
   static const bool legacy = [] { const char* e = getenv("YMP_ATTN_LEGACY"); return e && e[0] == '1'; }();
   const bool dropped = a->drop.rng && a->drop.p > 0.f;
   YMP_CHECK_ARG(!dropped || a->drop.p < 1.f, "ymp_attn_fwd: dropout p must be < 1");
-  if (a->s_q == 1 && a->mask == YMP_MASK_NONE && a->total_rows == 0 && !dropped && a->head_dim != 88 && a->head_dim != 128 && !legacy) {
+  const bool decode = a->s_q == 1 && a->mask == YMP_MASK_NONE && a->total_rows == 0 && !dropped && a->head_dim != 88 && a->head_dim != 128;
+  YMP_CHECK_ARG(!a->kv_rows || (decode && a->ld_kv_rows >= a->s_kv),
+                "ymp_attn_fwd: kv_rows needs the single-query decoding kernel (s_q == 1, mask none, no dropout, no total_rows, "
+                "head_dim 64 / 80 / 96) and ld_kv_rows >= s_kv");
+  if (decode && (!legacy || a->kv_rows)) {
     g_attn_path = YMP_ATTN_PATH_DECODE;   // one query row per sequence: the streaming kernel (also follows s_kv_dev)
     switch (a->head_dim) {
       case 64: return launch_decode<64>(p, st);
@@ -902,6 +918,7 @@ extern "C" int ymp_attn_bwd(const ymp_attn_bwd_args* b, void* stream) {
   YMP_CHECK_ARG(a->o && a->lse && b->dout && b->dq && b->dk && b->dv && b->delta_ws, "ymp_attn_bwd: null o/lse/dout/dq/dk/dv/delta_ws");
   YMP_CHECK_ARG(b->lddo % 8 == 0 && b->lddq % 8 == 0 && b->lddk % 8 == 0 && b->lddv % 8 == 0, "ymp_attn_bwd: grad row strides must be multiples of 8");
   YMP_CHECK_ARG(!a->s_kv_dev, "ymp_attn_bwd: s_kv_dev is forward only");
+  YMP_CHECK_ARG(!a->kv_rows, "ymp_attn_bwd: kv_rows is served by the single-query decoding kernel only");
   p.dout = (const __nv_bfloat16*)b->dout; p.dq = (__nv_bfloat16*)b->dq; p.dk = (__nv_bfloat16*)b->dk; p.dv = (__nv_bfloat16*)b->dv;
   p.delta = b->delta_ws;
   p.lddo = b->lddo; p.hsdo = b->do_head_stride;

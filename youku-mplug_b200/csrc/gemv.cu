@@ -15,6 +15,7 @@
 //   * partial sums meet in shared memory; lane (g, t) of the slice-0 warp owns (row g, columns n0+2t, n0+2t+1) and applies
 //       v = acc + bias[n] ; v = gelu(v) (optional) ; v += residual[m, n] (bf16 or fp32) ; store bf16 or fp32
 //     (+ an optional second bf16 copy at a device-side row offset: the KV-cache row of the new token).
+// 9..64 rows (batched beam search) run on gemm_skinny_wide_kernel below: the same layout with up to four m16 row tiles.
 // Algorithmic bytes per call: N*K*2 (weights) + M*(K + N)*2..4.
 #include "common.h"
 #include "ptx.cuh"
@@ -219,13 +220,131 @@ __global__ void __launch_bounds__(SK_WARPS * 32, (LN ? 2 : 1)) gemm_skinny_kerne
   }
 }
 
+// 9 <= M <= 64 rows (batched beam search: n_samples x beam rows).  Same CTA / warp / K-slice layout as the kernel above
+// (chosen from N and K only), same k permutation, same MMA sequence per k-block and the same cross-warp reduction order,
+// so row r of the result depends on row r of x alone, bit for bit, at any M.  The rows are MT m16 tiles of the A
+// operand: lane (g, t) feeds rows 16i + g and 16i + 8 + g of tile i, and every tile reuses the weight fragments the lane
+// already holds - the weights are still read once.  Only the weights are double-buffered; the activations (L1/L2
+// resident) are loaded for the current batch, which keeps the register budget at two CTAs per SM.
+__device__ __forceinline__ void mma16816_bf16_full(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
+                                                   uint32_t b1) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+}
+
+__device__ __forceinline__ void skinny_store(const SkinnyParams& p, int m, int n, float v) {
+  if (p.bias) v += __bfloat162float(p.bias[n]);
+  if (p.act == YMP_ACT_GELU_TANH) v = gelu_tanh(v);
+  else if (p.act == YMP_ACT_GELU_ERF) v = gelu_erf(v);
+  if (p.residual)
+    v += p.res_f32 ? reinterpret_cast<const float*>(p.residual)[(size_t)m * p.ldr + n]
+                   : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(p.residual)[(size_t)m * p.ldr + n]);
+  if (p.out_f32) reinterpret_cast<float*>(p.y)[(size_t)m * p.ldy + n] = v;
+  else reinterpret_cast<__nv_bfloat16*>(p.y)[(size_t)m * p.ldy + n] = __float2bfloat16(v);
+  if (p.y2) p.y2[(long long)m * p.ldy2 + *p.y2_off * p.y2_stride + n] = __float2bfloat16(v);
+}
+
+constexpr int SK_WIDE_MAXM = 64, SK_WIDE_UNROLL = 4;
+
+template <int MT>
+__global__ void __launch_bounds__(SK_WARPS * 32, 2) gemm_skinny_wide_kernel(const SkinnyParams p) {
+  constexpr int U = SK_WIDE_UNROLL;
+  __shared__ float part[SK_WARPS][MT * 128];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int g = lane >> 2, t = lane & 3;
+  const int ks = p.ksplit, kpart = warp % ks, tile = blockIdx.x * (SK_WARPS / ks) + warp / ks;
+  const int n0 = tile * SK_TILE_N;
+  const bool live = n0 < p.N;
+  float acc[MT][4];
+#pragma unroll
+  for (int i = 0; i < MT; ++i) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.f;
+  griddep_launch();
+  if (live) {
+    const int nchunk = p.K >> 3, nblk = (nchunk + 3) >> 2;
+    const int b_lo = (int)((long)nblk * kpart / ks), b_hi = (int)((long)nblk * (kpart + 1) / ks);
+    const uint4* wr = reinterpret_cast<const uint4*>(p.w + (size_t)min(n0 + g, p.N - 1) * p.ldw);
+    const uint4* xr[MT][2];
+    bool xrow[MT][2];
+#pragma unroll
+    for (int i = 0; i < MT; ++i)
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int m = 16 * i + 8 * h + g;
+        xrow[i][h] = m < p.M;
+        xr[i][h] = reinterpret_cast<const uint4*>(p.x + (size_t)min(m, p.M - 1) * p.ldx);
+      }
+    uint4 wv[U];
+    auto fetch_w = [&](int b, uint4 (&wd)[U]) {
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int c = (b + u) * 4 + t;
+        wd[u] = ((b + u) < b_hi && c < nchunk) ? ld_nc_v4(wr + c) : make_uint4(0, 0, 0, 0);
+      }
+    };
+    fetch_w(b_lo, wv);
+    griddep_wait();
+    for (int b = b_lo; b < b_hi; b += U) {
+      uint4 wn[U];
+      fetch_w(b + U, wn);
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int c = (b + u) * 4 + t;
+        const bool in = (b + u) < b_hi && c < nchunk;
+#pragma unroll
+        for (int i = 0; i < MT; ++i) {
+          const uint4 x0 = (in && xrow[i][0]) ? __ldg(xr[i][0] + c) : make_uint4(0, 0, 0, 0);
+          const uint4 x1 = (in && xrow[i][1]) ? __ldg(xr[i][1] + c) : make_uint4(0, 0, 0, 0);
+          mma16816_bf16_full(acc[i], x0.x, x1.x, x0.y, x1.y, wv[u].x, wv[u].y);
+          mma16816_bf16_full(acc[i], x0.z, x1.z, x0.w, x1.w, wv[u].z, wv[u].w);
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) wv[u] = wn[u];
+    }
+  } else {
+    griddep_wait();
+  }
+  // acc[i][2h + e] = (row 16i + 8h + g, column n0 + 2t + e) summed over this warp's K slice
+  if (ks > 1) {
+#pragma unroll
+    for (int i = 0; i < MT; ++i)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) part[warp][i * 128 + 4 * lane + e] = acc[i][e];
+    __syncthreads();
+    if (kpart == 0)
+      for (int j = 1; j < ks; ++j)
+#pragma unroll
+        for (int i = 0; i < MT; ++i)
+#pragma unroll
+          for (int e = 0; e < 4; ++e) acc[i][e] += part[warp + j][i * 128 + 4 * lane + e];
+  }
+  if (live && kpart == 0) {
+#pragma unroll
+    for (int i = 0; i < MT; ++i)
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int m = 16 * i + 8 * h + g;
+        if (m >= p.M) continue;
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int n = n0 + 2 * t + e;
+          if (n < p.N) skinny_store(p, m, n, acc[i][2 * h + e]);
+        }
+      }
+  }
+}
+
 }  // namespace ymp
 
 using namespace ymp;
 
-extern "C" int ymp_gemm_skinny(const ymp_gemm_skinny_args* a, void* stream) {
+// ymp_gemm_skinny (M <= 8) and ymp_gemm_skinny_batch (M <= 64): one implementation, the same kernel for M <= 8
+static int gemm_skinny_call(const ymp_gemm_skinny_args* a, void* stream, int max_m) {
   YMP_CHECK_ARG(a && a->x && a->w && a->y, "ymp_gemm_skinny: null pointer");
-  YMP_CHECK_ARG(a->M >= 1 && a->M <= SK_MAXM && a->N > 0 && a->K > 0 && a->K % 8 == 0, "ymp_gemm_skinny: needs 1 <= M <= 8, K %% 8 == 0 (M=%d K=%d)", a->M, a->K);
+  YMP_CHECK_ARG(a->M >= 1 && a->M <= max_m && a->N > 0 && a->K > 0 && a->K % 8 == 0, "ymp_gemm_skinny: needs 1 <= M <= %d, K %% 8 == 0 (M=%d K=%d)", max_m, a->M, a->K);
+  YMP_CHECK_ARG(!a->ln_out || a->M <= SK_MAXM, "ymp_gemm_skinny: the fused LayerNorm needs M <= 8 (M=%d)", a->M);
   YMP_CHECK_ARG(a->ldx % 8 == 0 && a->ldw % 8 == 0 && a->ldx >= a->K && a->ldw >= a->K && aligned16(a->x) && aligned16(a->w), "ymp_gemm_skinny: x / w rows must be 16-byte aligned");
   YMP_CHECK_ARG(a->act >= 0 && a->act <= 2, "ymp_gemm_skinny: bad act");
   SkinnyParams p;
@@ -252,6 +371,15 @@ extern "C" int ymp_gemm_skinny(const ymp_gemm_skinny_args* a, void* stream) {
   const int blocks = (tiles + tiles_per_cta - 1) / tiles_per_cta;
   static const int unroll = [] { const char* e = getenv("YMP_SKINNY_UNROLL"); return e ? atoi(e) : 4; }();
   cudaStream_t st = (cudaStream_t)stream;
+  if (a->M > SK_MAXM) {   // same grid, one to four m16 row tiles per warp
+    const int mt = (a->M + 15) / 16;
+    if (mt == 1) launch_k(gemm_skinny_wide_kernel<1>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
+    else if (mt == 2) launch_k(gemm_skinny_wide_kernel<2>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
+    else if (mt == 3) launch_k(gemm_skinny_wide_kernel<3>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
+    else launch_k(gemm_skinny_wide_kernel<4>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
+    YMP_LAUNCH_CHECK();
+    return YMP_OK;
+  }
   if (ln) launch_k(gemm_skinny_kernel<4, true>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
   else if (unroll == 8) launch_k(gemm_skinny_kernel<8, false>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
   else if (unroll == 2) launch_k(gemm_skinny_kernel<2, false>, dim3(blocks), dim3(SK_WARPS * 32), 0, st, p);
@@ -259,3 +387,6 @@ extern "C" int ymp_gemm_skinny(const ymp_gemm_skinny_args* a, void* stream) {
   YMP_LAUNCH_CHECK();
   return YMP_OK;
 }
+
+extern "C" int ymp_gemm_skinny(const ymp_gemm_skinny_args* a, void* stream) { return gemm_skinny_call(a, stream, SK_MAXM); }
+extern "C" int ymp_gemm_skinny_batch(const ymp_gemm_skinny_args* a, void* stream) { return gemm_skinny_call(a, stream, SK_WIDE_MAXM); }

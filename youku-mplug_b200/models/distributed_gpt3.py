@@ -301,6 +301,17 @@ class DistributedGPT3_Caption(_PrefixModelBase):
             res.append(out.sequences.cpu())
         return res
 
+    @torch.no_grad()
+    def generate_batch(self, image, text):
+        """What generate(image, text) returns - the same list of [1, len] CPU LongTensors, same stop token and prompt
+        lengths - with the visual prefix computed once and the clips decoded together (DistributedGPT3.beam_search_batch:
+        the beams of up to 64 // beam clips of equal prompt length share every decoding step)."""
+        _, _, _, query_features = self.visual_prefix(image)
+        eos = self.tokenizer.tokenizer.eos if self.tokenizer is not None else self.text_decoder.config.eod_id
+        out = self.text_decoder.beam_search_batch(text.input_ids, query_embeds=query_features,
+                                                  prompt_length=text.attention_mask.sum(-1) - 1, stop_token=eos)
+        return [o.sequences.cpu() for o in out]
+
 
 class _PromptClsBase(_PrefixModelBase):
     """Shared forward pieces of DistributedGPT3_Cls (:431-657) and DistributedGPT3_Retrieval_Cls (:988-1218):

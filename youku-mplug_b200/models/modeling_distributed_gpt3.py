@@ -453,6 +453,164 @@ def run_beam_search(step, reorder, tokens, prompt_length, n_query, *, beam_size,
                     scores=torch.stack([torch.as_tensor(sc, device=dev).reshape(-1)[0] for sc, _, _ in best], dim=0))
 
 
+def beam_chunks(prompt_lengths, per_chunk):
+    """(prompt_length, sample indices) of every decode batch of run_beam_search_batch: the samples grouped by prompt
+    length (groups in order of first appearance), each group cut into chunks of at most per_chunk samples."""
+    groups = {}
+    for i, p in enumerate(prompt_lengths):
+        groups.setdefault(int(p), []).append(i)
+    for p, idx in groups.items():
+        for c in range(0, len(idx), per_chunk):
+            yield p, idx[c:c + per_chunk]
+
+
+def run_beam_search_batch(step, reorder, tokens, prompt_lengths, n_query, *, beam_size, num_return_gen, stop_token,
+                          tokens_to_generate, max_position_embeddings, max_rows=64):
+    """run_beam_search for every sample of tokens [B, L] at once: element i of the returned list equals
+    run_beam_search on sample i alone (same ranking, same stop-token rule, same BeamHypotheses calls).
+
+    The samples are decoded in chunks of n = max_rows // beam_size samples of equal prompt length (beam_chunks); a short
+    chunk is padded to n with copies of its first sample, whose results are dropped, so every chunk has the same shape.
+    Chunk row j * beam_size + b is beam b of sample samples[j].
+      step(samples, new_tokens [n * beam, k], first) -> next-token logits [n * beam, V] (first: new_tokens is the whole
+          prompt and the callback also feeds the visual prefix of samples[j] to its rows)
+      reorder(idx) -> row r continues the history of row idx[r] (int64 [n * beam], rows of the chunk)
+    One log_softmax over all rows, one top-k over [n, beam * V] and one device-to-host copy per step serve every sample.
+    A sample that has finished keeps its rows: they are fed its stop token, never reordered, and their logits ignored."""
+    dev = tokens.device
+    beam = beam_size
+    per = max_rows // beam
+    if per < 1:
+        raise ValueError(f"beam_size {beam} > max_rows {max_rows}")
+    plens = [int(p) for p in torch.as_tensor(prompt_lengths).reshape(-1).tolist()]
+    assert len(plens) == tokens.size(0)
+    final_len = min(tokens.size(1) + tokens_to_generate, max_position_embeddings)
+    results = [None] * tokens.size(0)
+    for plen, idx in beam_chunks(plens, per):
+        if plen >= final_len:
+            raise ValueError('context length + tokens_to_generate too large')
+        samples = idx + [idx[0]] * (per - len(idx))
+        n, R = per, per * beam
+        toks = torch.cat((tokens[samples].cpu(), torch.full((n, tokens_to_generate), stop_token, dtype=torch.long)), dim=-1)
+        toks = toks.repeat_interleave(beam, dim=0)                     # [R, L + tokens_to_generate], host
+        pools = [BeamHypotheses(beam) for _ in range(n)]
+        done = [False] * n
+        scores = torch.zeros(R, 1, dtype=torch.float32, device=dev)
+        host_scores = torch.zeros(R, dtype=torch.float32)
+        prev = 0
+        ctx = plen
+        for ctx in range(plen, final_len):
+            first = ctx == plen
+            logits = step(samples, toks[:, prev:ctx].to(dev), first)
+            vocab = logits.size(-1)
+            cand = torch.log_softmax(logits.float(), dim=-1) + scores
+            flat = cand.view(n, beam, vocab)[:, 0] if first else cand.view(n, beam * vocab)   # identical beams at first
+            top_dev, top_i = torch.topk(flat, 2 * beam, dim=-1)
+            host = torch.cat([top_dev.view(torch.int32), top_i.to(torch.int32)], dim=1).cpu()
+            top_s, top_i = host[:, :2 * beam].view(torch.float32), host[:, 2 * beam:].long()
+            keep = list(range(R))
+            for j in range(n):
+                if done[j]:
+                    continue
+                ranked_scores = top_s[j]
+                beam_of, word_of = torch.div(top_i[j], vocab, rounding_mode='floor').tolist(), (top_i[j] % vocab).tolist()
+                survivors = []
+                for rank, (word, b) in enumerate(zip(word_of, beam_of)):
+                    if word == stop_token:
+                        if rank >= beam:
+                            continue
+                        # the score is divided where run_beam_search divides it (on the logits' device), for the same bits
+                        pools[j].add(toks[j * beam + b].clone(), top_dev[j, rank], ctx + 1 - plen)
+                    else:
+                        survivors.append((word, ranked_scores[rank], b))
+                    if len(survivors) == beam:
+                        break
+                if pools[j].is_done(ranked_scores.max().item(), ctx + 1 - plen):
+                    done[j] = True
+                    continue
+                rows = [j * beam + b for _, _, b in survivors]
+                keep[j * beam:(j + 1) * beam] = rows
+                block = toks[rows, :]
+                block[:, ctx] = torch.tensor([w for w, _, _ in survivors], dtype=torch.long)
+                toks[j * beam:(j + 1) * beam] = block
+                host_scores[j * beam:(j + 1) * beam] = torch.stack([sc for _, sc, _ in survivors])
+            if all(done):
+                break
+            scores = host_scores.view(R, 1).to(dev)
+            reorder(torch.tensor(keep, dtype=torch.long, device=dev))
+            prev = ctx
+        for j, i in enumerate(idx):
+            pool = pools[j]
+            if not done[j]:
+                for b in range(beam):
+                    pool.add(toks[j * beam + b].clone(), scores[j * beam + b], ctx + 1 - plen)
+            best = sorted(pool.beams, key=lambda x: float(x[0]), reverse=True)[:min(num_return_gen, len(pool.beams))]
+            results[i] = AttrDict(sequences=torch.stack([h for _, h, _ in best], dim=0).to(dev),
+                                  scores=torch.stack([torch.as_tensor(sc, device=dev).reshape(-1)[0] for sc, _, _ in best], dim=0))
+    return results
+
+
+class _BeamBatchDecoder:
+    """Decode callbacks of DistributedGPT3.beam_search_batch over one ymp.engine.BeamBatchCache of n x beam rows.
+    The first step prefills every sample into its own block of rows with exactly the calls DistributedGPT3._decode
+    makes for a single beam search (so the cached prefix and the first logits are the same bits); every later step is
+    one replay of the captured TokenStep over all rows, the decode attention reading its keys through the cache's row
+    table, and a reorder rewrites table entries only."""
+
+    def __init__(self, model, query_embeds, beam, n, max_len, device):
+        from ymp import engine
+        self.model, self.qe, self.beam, self.n = model, query_embeds, beam, n
+        keys, params = model._param_list()
+        self.params = params
+        self.W = {k: YF.as_bf16(p) for k, p in zip(keys, params)}
+        # one cache (and its captured step) per shape, kept apart from the per-sample pool so that alternating with
+        # generate() recaptures nothing
+        key = (n * beam, beam, max_len, str(device))
+        pool = model.__dict__.setdefault("_beam_batch_pool", {})
+        if key not in pool:
+            pool.clear()
+            pool[key] = engine.BeamBatchCache(model.config.engine_cfg(), n, beam, max_len, device)
+        self.cache = pool[key]
+
+    def _token_step(self, emb_dtype):
+        from ymp import engine
+        params = self.params
+        sig = (params[0].data_ptr(), params[-1].data_ptr(), sum(p._version for p in params))
+        ts = self.cache.token
+        if ts is None or ts.sig != sig:
+            static = all(p.dtype == torch.bfloat16 or not p.requires_grad for p in params)
+            ts = self.cache.token = engine.TokenStep(self.cache, self.W, emb_dtype, sig, static)
+        elif not ts.static:
+            ts.W = self.W
+        return ts
+
+    def step(self, samples, new_tokens, first):
+        from ymp import engine, ops
+        c, beam, W = self.cache, self.beam, self.W
+        emb = self.model.dist_model.language_model.embedding.word_embeddings(new_tokens)   # [R, k, H]
+        R, n, H = emb.shape
+        if not first:
+            _, logits = self._token_step(emb.dtype).run(emb.reshape(R, H))
+            return logits
+        c.reset()
+        pos = W[engine.GPT + "embedding.position_embeddings.weight"]
+        out = []
+        for j, s in enumerate(samples):
+            ie = emb[j * beam:(j + 1) * beam]
+            if self.qe is not None:
+                ie = torch.cat([self.qe[s:s + 1].repeat(beam, 1, 1).to(ie.dtype), ie], dim=1)
+            k = ie.size(1)
+            x = (ie.float() + pos[0:k][None].float()).reshape(beam * k, H).contiguous()
+            hid = engine.gpt_decode(W, x, c.block(j), k)
+            out.append(ops.gemm(hid, W[engine.GPT + "embedding.word_embeddings.weight"]).float())
+        c._set_len(k)
+        c.start_table(k)
+        return torch.cat(out)
+
+    def reorder(self, idx):
+        self.cache.reorder_table(idx)
+
+
 class GPT3Model(nn.Module):
     """Parameter container with the reference's names: language_model.{embedding,encoder}...."""
 
@@ -644,6 +802,29 @@ class DistributedGPT3(nn.Module):
         return run_beam_search(step, reorder, tokens, prompt_length, nq, beam_size=beam_size, num_return_gen=num_return_gen,
                                stop_token=stop_token, tokens_to_generate=cfg.tokens_to_generate,
                                max_position_embeddings=cfg.max_position_embeddings)
+
+    @torch.no_grad()
+    def beam_search_batch(self, tokens, query_embeds=None, prompt_length=None, beam_size=5, num_return_gen=1, stop_token=None):
+        """beam_search for every sample of tokens [B, L] (visual prefixes query_embeds [B, Q, H], prompt lengths
+        prompt_length [B]): a list of B Dict(sequences [n, len], scores [n]), element i equal to beam_search on sample i.
+        Samples of equal prompt length share one decoding step: chunks of 64 // beam_size samples, each step one replay
+        of the captured token step over all their beams (one weight stream instead of one per sample).  With
+        beam_size <= 8 the logits are the bits of the per-sample path."""
+        from ymp import ops
+        cfg = self.config
+        B = tokens.size(0)
+        if prompt_length is None:
+            prompt_length = torch.full((B,), tokens.size(1), dtype=torch.long)
+        prompt_length = torch.as_tensor(prompt_length).reshape(-1)
+        if stop_token is None:
+            stop_token = cfg.eod_id
+        nq = 0 if query_embeds is None else query_embeds.size(1)
+        final_len = min(tokens.size(1) + cfg.tokens_to_generate, cfg.max_position_embeddings)
+        per = ops.SKINNY_WIDE_MAX_ROWS // beam_size
+        dec = _BeamBatchDecoder(self, query_embeds, beam_size, per, final_len + nq, tokens.device)
+        return run_beam_search_batch(dec.step, dec.reorder, tokens, prompt_length, nq, beam_size=beam_size,
+                                     num_return_gen=num_return_gen, stop_token=stop_token, tokens_to_generate=cfg.tokens_to_generate,
+                                     max_position_embeddings=cfg.max_position_embeddings, max_rows=per * beam_size)
 
     @torch.no_grad()
     def generate(self, tokens, do_sample=True, termination_id=None, *args, **kwargs):

@@ -670,12 +670,65 @@ class KVCache:
         v.copy_(v.index_select(1, idx))
 
 
+class _RowBlock:
+    """Rows [r0, r0 + rows) of a KVCache, seen as a cache of their own by gpt_decode (the per-sample prefill of a batched
+    beam search writes one sample's beams into its block with exactly the call a single beam search makes)."""
+
+    def __init__(self, cache, r0, rows):
+        ML = cache.max_len
+        self.g, self.B, self.max_len, self.len = cache.g, rows, ML, 0
+        self.qkv = [t[r0 * ML:(r0 + rows) * ML] for t in cache.qkv]
+
+    def _set_len(self, n):
+        self.len = n
+
+
+class BeamBatchCache(KVCache):
+    """KV cache of a batch of beam searches: R = n_samples x beam rows, sample i owning rows [i*beam, (i+1)*beam).
+    Attention finds key j of row r through the int32 device table `table[r, j]` (a cache row index), so a beam reorder
+    moves table entries - `table[:, :len] = table[parent, :len]`, a few kilobytes - instead of every cached position of
+    every layer.  The new token of row r is still written to slot r * max_len + len: no table entry refers to it before
+    that step (entries at and past `len` are the identity), so cached K/V is never rewritten.  After the prefill every
+    beam of a sample reads its prefix positions from the sample's beam-0 rows (`start_table`), which keeps one copy of
+    each prefix in L2 instead of `beam`."""
+
+    def __init__(self, gcfg, n_samples, beam, max_len, device):
+        super().__init__(gcfg, n_samples * beam, max_len, device)
+        self.n_samples, self.beam = n_samples, beam
+        self.table = torch.empty((self.B, max_len), device=device, dtype=torch.int32)
+        self.start_table(0)
+
+    def block(self, i):
+        """Sample i's rows as a cache of `beam` sequences (for its prefill)."""
+        return _RowBlock(self, i * self.beam, self.beam)
+
+    def start_table(self, prefix_len):
+        """Identity table, except that positions < prefix_len of every row read the rows of its sample's beam 0."""
+        R, ML = self.B, self.max_len
+        rows = torch.arange(R, dtype=torch.int64)
+        src = rows.clone()
+        src_prefix = (rows // self.beam) * self.beam
+        tab = src[:, None] * ML + torch.arange(ML, dtype=torch.int64)[None, :]
+        tab[:, :prefix_len] = src_prefix[:, None] * ML + torch.arange(prefix_len, dtype=torch.int64)[None, :]
+        self.table.copy_(tab.to(torch.int32))
+
+    def reorder_table(self, idx):
+        """Row r continues the history of row idx[r] (idx: int64 device tensor [R])."""
+        assert idx.numel() == self.B
+        if self.len == 0:
+            return
+        t = self.table[:, :self.len]
+        t.copy_(t.index_select(0, idx))
+
+
 class TokenStep:
     """The single-token decoding step (n == 1, cache not empty) for at most ops.SKINNY_MAX_ROWS sequences, as ONE CUDA
     graph: every linear is a skinny GEMM (one pass over its weights, csrc/gemv.cu), the new K/V row goes into the cache
     at the device-side position `len_idx`, attention reads `len1` keys (ymp_attn_args.s_kv_dev), and the graph ends by
     advancing both counters - so one captured graph serves every position of every generate() call that reuses this
-    cache.  ~8 kernels per layer; the latency floor is the weight stream (2.6 GB at 1.3B)."""
+    cache.  ~8 kernels per layer; the latency floor is the weight stream (2.6 GB at 1.3B).
+    Over a BeamBatchCache the same step serves up to ops.SKINNY_WIDE_MAX_ROWS rows (a batch of beam searches), the
+    decode attention reading its keys through the cache's row table."""
 
     def __init__(self, cache, W, emb_dtype, sig=None, static=True):
         """sig: anything that changes when the weight tensors behind W move; static: W may be captured (raw pointers)."""
@@ -713,7 +766,9 @@ class TokenStep:
         # input (one kernel boundary less per sub-layer).  Off by default: measured neutral on B200 (captured step 1.466
         # vs 1.438 ms, profiles/r02p_decode_ab.log) - the ticket + three L2 round trips of the tail cost what the
         # stand-alone kernel and its launch gap cost.
-        fused_ln = os.environ.get("YMP_DECODE_FUSED_LN", "0") == "1"
+        fused_ln = os.environ.get("YMP_DECODE_FUSED_LN", "0") == "1" and B <= ops.SKINNY_MAX_ROWS
+        kv_rows = getattr(c, "table", None)   # BeamBatchCache: keys through the per-row table
+        skinny = ops.gemm_skinny if B <= ops.SKINNY_MAX_ROWS else ops.gemm_skinny_batch
 
         def ln_of(prefix):
             return (W[prefix + ".weight"], W[prefix + ".bias"], g.eps, self.ticket)
@@ -721,9 +776,9 @@ class TokenStep:
         def gemm_ln(a, wname, residual, ln_prefix):
             """fp32 residual-stream GEMM followed by the LayerNorm of its complete result: (y, LN(y))."""
             if fused_ln:  # the LayerNorm is computed by the GEMM's last CTA
-                return ops.gemm_skinny(a, W[wname + ".weight"], bias=W[wname + ".bias"], residual=residual, out_dtype=torch.float32,
+                return skinny(a, W[wname + ".weight"], bias=W[wname + ".bias"], residual=residual, out_dtype=torch.float32,
                                        ln=ln_of(ln_prefix))
-            y = ops.gemm_skinny(a, W[wname + ".weight"], bias=W[wname + ".bias"], residual=residual, out_dtype=torch.float32)
+            y = skinny(a, W[wname + ".weight"], bias=W[wname + ".bias"], residual=residual, out_dtype=torch.float32)
             return y, ops.layernorm_fwd(y, W[ln_prefix + ".weight"], W[ln_prefix + ".bias"], g.eps, stats=False)[0]
 
         ln1, _, _ = ops.layernorm_fwd(x, W[f"{GPT}encoder.layers.0.input_layernorm.weight"], W[f"{GPT}encoder.layers.0.input_layernorm.bias"],
@@ -733,19 +788,19 @@ class TokenStep:
             st = self.stage
             buf = c.qkv[i]
             # [q|k|v] of the new token: into the staging rows (q for this step) and into cache row b*ML + len (k, v)
-            ops.gemm_skinny(ln1, W[pre + "self_attention.query_key_value.weight"], bias=W[pre + "self_attention.query_key_value.bias"],
+            skinny(ln1, W[pre + "self_attention.query_key_value.weight"], bias=W[pre + "self_attention.query_key_value.bias"],
                             out=st, out2=buf, out2_row_stride=ML, out2_off=c.len_idx)
             att = torch.empty((B, H), device=x.device, dtype=bf16)
             q = TView(st, 0, 3 * hd, ops.dense_map(1))
             k, v = TView(buf, hd, 3 * hd, mkv), TView(buf, 2 * hd, 3 * hd, mkv)
             ops.attn_fwd(q, k, v, TView(att, 0, hd, ops.dense_map(1)), n_seq=B, n_heads=g.heads, head_dim=hd, s_q=1, s_kv=ML,
-                         causal=False, scale=g.scale, s_kv_dev=c.len1)
+                         causal=False, scale=g.scale, s_kv_dev=c.len1, kv_rows=kv_rows)
             x1, ln2 = gemm_ln(att, pre + "self_attention.dense", x, pre + "post_attention_layernorm")
-            h = ops.gemm_skinny(ln2, W[pre + "mlp.dense_h_to_4h.weight"], bias=W[pre + "mlp.dense_h_to_4h.bias"], act=ACT_GELU_TANH)
+            h = skinny(ln2, W[pre + "mlp.dense_h_to_4h.weight"], bias=W[pre + "mlp.dense_h_to_4h.bias"], act=ACT_GELU_TANH)
             nxt = f"{GPT}encoder.layers.{i + 1}.input_layernorm" if i + 1 < g.layers else GPT + "encoder.final_layernorm"
             x, ln1 = gemm_ln(h, pre + "mlp.dense_4h_to_h", x1, nxt)
         hid = ln1
-        logits = ops.gemm_skinny(hid, W[GPT + "embedding.word_embeddings.weight"], out_dtype=torch.float32)
+        logits = skinny(hid, W[GPT + "embedding.word_embeddings.weight"], out_dtype=torch.float32)
         c.len_idx += 1
         c.len1 += 1
         return hid, logits

@@ -84,7 +84,7 @@ class AttnArgs(C.Structure):
         ("map_q", SeqMap), ("map_kv", SeqMap), ("map_o", SeqMap),
         ("n_seq", c_i32), ("n_heads", c_i32), ("head_dim", c_i32), ("s_q", c_i32), ("s_kv", c_i32),
         ("mask", c_i32), ("mask_block", c_i32), ("total_rows", C.c_int64), ("scale", C.c_float),
-        ("drop", DropoutSpec), ("s_kv_dev", c_vp),
+        ("drop", DropoutSpec), ("s_kv_dev", c_vp), ("kv_rows", c_vp), ("ld_kv_rows", c_i32),
     ]
 
 
@@ -166,6 +166,7 @@ def _declare(name, argstruct):
 
 _gemm = _declare("ymp_gemm", GemmArgs)
 _gemm_skinny = _declare("ymp_gemm_skinny", GemmSkinnyArgs)
+_gemm_skinny_batch = _declare("ymp_gemm_skinny_batch", GemmSkinnyArgs)
 _ln_fwd = _declare("ymp_layernorm_fwd", LayerNormArgs)
 _ln_bwd = _declare("ymp_layernorm_bwd", LayerNormBwdArgs)
 _attn_fwd = _declare("ymp_attn_fwd", AttnArgs)

@@ -114,19 +114,32 @@ def gemm(a, b, *, a_t=False, b_t=False, bias=None, residual=None, act=ACT_NONE, 
     return out
 
 
-SKINNY_MAX_ROWS = 8
+SKINNY_MAX_ROWS = 8        # one beam search (the captured per-sample decoding step); the fused LayerNorm stops here
+SKINNY_WIDE_MAX_ROWS = 64  # a batch of beam searches
 
 
-def gemm_skinny(x, w, *, bias=None, residual=None, act=ACT_NONE, out=None, out_dtype=bf16, out2=None, out2_row_stride=0,
-                out2_off=None, ln=None):
+def gemm_skinny(x, w, **kw):
     """y[M, N] = act(x[M, K] @ w[N, K]^T + bias) + residual for M <= 8 rows (single-token decoding): one pass over
-    the weights on the HBM-bound kernel of csrc/gemv.cu instead of a mostly empty 128-row tensor-core tile.
+    the weights on the HBM-bound kernel of csrc/gemv.cu instead of a mostly empty 128-row tensor-core tile.  Row m of y
+    depends on row m of x only, bit for bit, whatever M is.  Keywords:
+    bias, residual, act, out, out_dtype: the epilogue and the result buffer / dtype.
     out2 [R, N] bf16 with out2_off (int64 device scalar): result row m is also written to out2 row
     m * out2_row_stride + out2_off (the KV-cache row at the device-side cache length).
     ln = (gamma, beta, eps, counter): also returns LN(y) [M, N] bf16, computed inside the same kernel by the CTA that
     finishes last (counter: uint32/int32 device scalar, zero at launch, reset by the kernel); result is then (y, ln_y)."""
+    return _skinny(L._gemm_skinny, "ymp_gemm_skinny", SKINNY_MAX_ROWS, x, w, **kw)
+
+
+def gemm_skinny_batch(x, w, **kw):
+    """gemm_skinny for up to 64 rows (ymp_gemm_skinny_batch): the step of a batch of beam searches.  Same keywords;
+    the fused LayerNorm `ln` still needs M <= 8.  Row m of the result has the bits gemm_skinny gives it."""
+    return _skinny(L._gemm_skinny_batch, "ymp_gemm_skinny_batch", SKINNY_WIDE_MAX_ROWS, x, w, **kw)
+
+
+def _skinny(entry, name, max_rows, x, w, *, bias=None, residual=None, act=ACT_NONE, out=None, out_dtype=bf16, out2=None,
+            out2_row_stride=0, out2_off=None, ln=None):
     _chk2d(x, "x"); _chk2d(w, "w")
-    assert x.dtype == bf16 and w.dtype == bf16 and x.shape[1] == w.shape[1] and x.shape[0] <= SKINNY_MAX_ROWS
+    assert x.dtype == bf16 and w.dtype == bf16 and x.shape[1] == w.shape[1] and x.shape[0] <= max_rows
     M, K, N = x.shape[0], x.shape[1], w.shape[0]
     if out is None:
         out = torch.empty((M, N), device=x.device, dtype=out_dtype)
@@ -155,7 +168,7 @@ def gemm_skinny(x, w, *, bias=None, residual=None, act=ACT_NONE, out=None, out_d
         ln_out = torch.empty((M, N), device=x.device, dtype=bf16)
         a.ln_gamma, a.ln_beta, a.ln_out, a.ln_counter = gamma.data_ptr(), beta.data_ptr(), ln_out.data_ptr(), counter.data_ptr()
         a.ld_ln, a.ln_eps = ln_out.stride(0), eps
-    L.call(L._gemm_skinny, a, "ymp_gemm_skinny")
+    L.call(entry, a, name)
     return out if ln is None else (out, ln_out)
 
 
@@ -239,7 +252,7 @@ class TView:
 
 
 def _attn_args(q, k, v, o, lse, n_seq, n_heads, head_dim, s_q, s_kv, causal, scale, mask_block=0, total_rows=0, drop=None,
-               s_kv_dev=None):
+               s_kv_dev=None, kv_rows=None):
     a = L.AttnArgs()
     a.q, a.k, a.v, a.o, a.lse = q.p, k.p, v.p, o.p, L.ptr(lse)
     a.ldq, a.ldk, a.ldv, a.ldo = q.ld, k.ld, v.ld, o.ld
@@ -252,16 +265,22 @@ def _attn_args(q, k, v, o, lse, n_seq, n_heads, head_dim, s_q, s_kv, causal, sca
     if s_kv_dev is not None:
         assert s_kv_dev.dtype == torch.int32 and s_kv_dev.is_cuda and s_kv_dev.numel() == 1
         a.s_kv_dev = s_kv_dev.data_ptr()
+    if kv_rows is not None:
+        assert kv_rows.dtype == torch.int32 and kv_rows.is_cuda and kv_rows.dim() == 2 and kv_rows.stride(1) == 1
+        assert kv_rows.shape[0] >= n_seq
+        a.kv_rows, a.ld_kv_rows = kv_rows.data_ptr(), kv_rows.stride(0)
     return a
 
 
 def attn_fwd(q, k, v, o, *, n_seq, n_heads, head_dim, s_q, s_kv, causal, scale, lse=None, mask_block=0,
-             total_rows=0, drop=None, s_kv_dev=None):
+             total_rows=0, drop=None, s_kv_dev=None, kv_rows=None):
     """q,k,v,o: TView.  Returns lse [n_seq, n_heads, s_q] fp32.  s_kv_dev: int32 device scalar, only the first
-    min(s_kv, s_kv_dev) keys exist (the captured decoding step)."""
+    min(s_kv, s_kv_dev) keys exist (the captured decoding step).  kv_rows: int32 device table [n_seq, >= s_kv]: key j
+    of sequence s is row kv_rows[s, j] of k's and v's tensors (k.m is then unused; single-query decoding only)."""
     if lse is None:
         lse = torch.empty((n_seq, n_heads, s_q), device=q.t.device, dtype=torch.float32)
-    a = _attn_args(q, k, v, o, lse, n_seq, n_heads, head_dim, s_q, s_kv, causal, scale, mask_block, total_rows, drop, s_kv_dev)
+    a = _attn_args(q, k, v, o, lse, n_seq, n_heads, head_dim, s_q, s_kv, causal, scale, mask_block, total_rows, drop, s_kv_dev,
+                   kv_rows)
     L.call(L._attn_fwd, a, "ymp_attn_fwd")
     return lse
 
